@@ -4,7 +4,7 @@ weak-label domain analysis -> repair-model inference -> (tid, attribute, current
 one synthetic N x K categorical table (config C4 of SURVEY.md section 8d).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--rows R] [--cols C] [--scaling strong|weak]
-                  [--impl reference]
+                  [--impl reference] [--dump-outputs DIR]
 
 N > 1 is launched by torchrun (one rank per GPU, NCCL).  Default = STRONG scaling: ONE R-row table,
 rows sharded R/N per GPU (BASELINE config 4); --scaling weak keeps R rows per GPU.  The only exchange
@@ -60,7 +60,17 @@ def parse_args():
     ap.add_argument("--verify-cells", type=int, default=50000)
     ap.add_argument("--trace", action="store_true",
                     help="one extra step with device-synchronised split points of the repair phase on stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the frame of the last one as DIR/<name>.npy (float64; see "
+                         "dump_outputs) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.warmup < 0:
+        ap.error("--warmup must not be negative")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs writes the frame of the b200 arm on one GPU: --impl b200 --gpus 1, no torchrun")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------
@@ -414,6 +424,47 @@ def verify_step(engine, table, res, out, models, k, n_sample, dist, seed=12345):
     return info
 
 
+DUMP_SAMPLE_ROWS = 1 << 22
+DUMP_MAX_CELLS = 1_500_000   # 4 float64 arrays of 48 MB at most: a dump stays under 64 MB
+DUMP_SEED = 20261017
+
+
+def dump_outputs(path, out, names, dom, n_rows):
+    """Writes the (tid, attribute, current_value, repaired) frame that one pass handed its caller, in
+    dictionary codes (-1 = NULL), as float64 arrays under `path`:
+      cells_per_attribute [K]          cells of the whole frame per attribute (table column order);
+      current_hist, repaired_hist [K, max(dom) + 1]
+                                       the whole frame's counts of each code per attribute (column 0 = NULL);
+      tid, attribute, current_value, repaired [m]
+                                       every cell of a fixed sample of DUMP_SAMPLE_ROWS table rows (drawn with
+                                       DUMP_SEED, so the same for every run of the same --rows), ordered by
+                                       (attribute, tid), at most DUMP_MAX_CELLS of them.
+    Inputs are seeded, so two builds that compute the same frame write identical files."""
+    os.makedirs(path, exist_ok=True)
+    k, width = len(names), max(dom) + 1
+    sampled = np.zeros(n_rows, dtype=bool)
+    sampled[np.random.default_rng(DUMP_SEED).choice(n_rows, size=min(DUMP_SAMPLE_ROWS, n_rows), replace=False)] = True
+    counts = np.zeros(k)
+    cur_hist, rep_hist = np.zeros((k, width)), np.zeros((k, width))
+    parts = []
+    col_of = {a: i for i, a in enumerate(names)}
+    for a, rows, cur, rep in out:
+        i = col_of[a]
+        rows, cur, rep = np.asarray(rows, dtype=np.int64), np.asarray(cur, dtype=np.int64), np.asarray(rep, dtype=np.int64)
+        counts[i] += len(rows)
+        cur_hist[i] += np.bincount(cur + 1, minlength=width)
+        rep_hist[i] += np.bincount(rep + 1, minlength=width)
+        keep = sampled[rows]
+        parts.append(np.stack([rows[keep], np.full(int(keep.sum()), i), cur[keep], rep[keep]]))
+    cells = np.concatenate(parts, axis=1) if parts else np.zeros((4, 0), dtype=np.int64)
+    cells = cells[:, np.lexsort((cells[0], cells[1]))][:, :DUMP_MAX_CELLS]
+    arrays = {"cells_per_attribute": counts, "current_hist": cur_hist, "repaired_hist": rep_hist,
+              "tid": cells[0], "attribute": cells[1], "current_value": cells[2], "repaired": cells[3]}
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
+    return {"dir": path, "sampled_cells": int(cells.shape[1]), "frame_cells": int(counts.sum())}
+
+
 # ---------------------------------------------------------------------------------------------
 # NUMA: a rank's host threads (Arrow ingest workers, the pinned chunk ring they fill) belong on the
 # CPU socket its GPU hangs off; 8 ranks sharing one socket's memory controllers is what cost the
@@ -461,7 +512,7 @@ def restore_affinity():
 # ---------------------------------------------------------------------------------------------
 # the other BASELINE.json configs: wall clock through the public API
 # ---------------------------------------------------------------------------------------------
-def other_configs(want, local):
+def other_configs(want, local, steps):
     import pandas as pd
     import torch
     from repair import (ConstraintErrorDetector, GaussianOutlierErrorDetector, NullErrorDetector, RepairModel, synth)
@@ -526,7 +577,6 @@ def other_configs(want, local):
         frozen = m.last_run["models"]
         timed_run(lambda: make().setFrozenModels(frozen))
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        steps = 3
         ev0.record()
         for _ in range(steps):
             t_inf, frame, mi = timed_run(lambda: make().setFrozenModels(frozen))
@@ -717,6 +767,8 @@ def b200_arm(args):
         return float(t[0]), float(t[1]), (engine.ctx.launch_count - l0), clocks, xs
 
     ms, ms_det, launches, clocks, exchanges = timed(args.steps, args.warmup)
+    # before any further pass: the frame of the last timed step borrows a staging buffer the next pass reuses
+    dumped = dump_outputs(args.dump_outputs, stats["last"][1], names, spec.dom, n) if args.dump_outputs else None
     cells = torch.tensor([stats["cells"], stats["out_rows"]], dtype=torch.int64, device=device)
     if dist is not None:
         dist.sum_(cells)
@@ -741,6 +793,8 @@ def b200_arm(args):
         "model_training_s": t_train, "forests": args.forests,
     }
     line["numa"] = numa
+    if dumped:
+        line["dump_outputs"] = dumped
     if dist is not None:
         line["exchanges_per_step"] = exchanges
 
@@ -889,7 +943,7 @@ def b200_arm(args):
             return frame
 
         api_step()                       # warm-up: allocator pools, the pinned chunk ring, page faults
-        e_steps = max(1, min(args.steps, 3))
+        e_steps = args.steps
         barrier()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
@@ -945,7 +999,7 @@ def b200_arm(args):
     if args.configs == "auto" and (world != 1 or args.rows != 100_000_000):
         want = []
     if want and rank == 0:
-        line["other_configs"] = other_configs(want, local)
+        line["other_configs"] = other_configs(want, local, args.steps)
 
     # ---- CPU baseline (rank 0, single GPU run only) -----------------------------------------------
     if rank == 0 and world == 1 and not args.no_cpu_baseline:

@@ -868,3 +868,35 @@ def test_bench_frame_comparison_catches_differences():
     assert not bench.frames_equal(frame(rep_a=(0, 2)), out, 100, names, table)        # a repaired value differs
     assert not bench.frames_equal(frame(ids_a=(101, 102)), out, 100, names, table)    # a row id differs
     assert not bench.frames_equal(frame(), out[:1], 100, names, table)                # an attribute is missing
+
+
+def test_bench_dump_outputs_is_float64_bounded_and_order_independent(tmp_path):
+    """bench.dump_outputs (--dump-outputs): whole-frame counts and per-attribute code histograms, plus every cell of
+    the seeded row sample sorted by (attribute, tid); the frame's order does not change the files."""
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    if root not in sys.path:
+        sys.path.insert(0, root)
+    import bench
+    names, dom, n = ["a", "b", "c"], [3, 2, 4], 10
+    out = [("a", np.array([1, 3], dtype=np.int32), np.array([-1, 2], dtype=np.int32), np.array([0, 1], dtype=np.int32)),
+           ("c", np.array([0, 9], dtype=np.int32), np.array([1, 3], dtype=np.int32), np.array([-1, 2], dtype=np.int32))]
+    info = bench.dump_outputs(str(tmp_path / "x"), out, names, dom, n)
+    got = {f[:-4]: np.load(str(tmp_path / "x" / f)) for f in os.listdir(str(tmp_path / "x"))}
+    assert info["frame_cells"] == 4 and info["sampled_cells"] == 4      # 10 rows: the sample is the whole table
+    assert all(a.dtype == np.float64 for a in got.values())
+    assert got["cells_per_attribute"].tolist() == [2, 0, 2]
+    assert got["current_hist"].shape == (3, 5) and got["current_hist"][0].tolist() == [1, 0, 0, 1, 0]
+    assert got["repaired_hist"][2].tolist() == [1, 0, 0, 1, 0]
+    assert got["tid"].tolist() == [1, 3, 0, 9] and got["attribute"].tolist() == [0, 0, 2, 2]
+    assert got["current_value"].tolist() == [-1, 2, 1, 3] and got["repaired"].tolist() == [0, 1, -1, 2]
+    bench.dump_outputs(str(tmp_path / "y"), [(a, r[::-1], c[::-1], p[::-1]) for a, r, c, p in out[::-1]], names, dom, n)
+    assert all(np.array_equal(a, np.load(str(tmp_path / "y" / (k + ".npy")))) for k, a in got.items())
+    # a larger table: the sample is a fixed subset of DUMP_SAMPLE_ROWS rows, the same in every run
+    big = bench.DUMP_SAMPLE_ROWS * 4
+    rows = np.arange(0, big, 2, dtype=np.int32)
+    zeros = np.zeros(len(rows), dtype=np.int32)
+    i1 = bench.dump_outputs(str(tmp_path / "p"), [("a", rows, zeros, zeros)], names, dom, big)
+    i2 = bench.dump_outputs(str(tmp_path / "q"), [("a", rows, zeros, zeros)], names, dom, big)
+    assert 0 < i1["sampled_cells"] < bench.DUMP_SAMPLE_ROWS and i1 == dict(i2, dir=i1["dir"])
+    assert np.array_equal(np.load(str(tmp_path / "p" / "tid.npy")), np.load(str(tmp_path / "q" / "tid.npy")))
