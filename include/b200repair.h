@@ -494,6 +494,26 @@ int dr_fd_map_build(dr_ctx* ctx, const int32_t* x_col, const uint32_t* x_mask, c
 int dr_tile_lut_fill(dr_ctx* ctx, int32_t* tile, int n_cols, int x_col, int y_col, const int32_t* cells,
                      int64_t n_cells, const int32_t* lut, int32_t lut_size, void* stream);
 
+/* ---- LOFOutlierErrorDetector: exact one-dimensional local outlier factor ---------------------------
+ * Replaces LOFOutlierErrorDetector (errors.py:302-312: sklearn LocalOutlierFactor per column).
+ *   col        device double[n], the whole column (NaN = NULL); when the table is sharded, the gathered
+ *              global column
+ *   k          neighbours, 1 <= k <= min(64, n - 1) (the detector uses min(20, n - 1))
+ *   bitmap     device uint32 words; only rows in [row_begin, row_begin + row_count) set bits, at bit
+ *              (row - row_begin); flagged iff lof > 1.5
+ *   out_lof    device double[n] (nullable): scores in row order; NaN when nothing was scored
+ *              (n < 2 or an all-NULL column)
+ *   out_flagged host int64 (nullable): number of rows flagged inside the range; non-NULL synchronises
+ *   workspace  device scratch of dr_lof_workspace_bytes(n) bytes (no allocation inside the call)
+ * Definition: NULL -> median of the non-NULL values (np.median), -0.0 -> +0.0; stable sort by
+ * (value, row); for sorted position i, the leftmost window [l, l + k] around i minimising
+ * max(s[i] - s[l], s[l + k] - s[i]) gives kdist and the neighbours; then scikit-learn's lrd / lof with
+ * the sums in ascending sorted position and round-to-nearest double arithmetic. */
+int64_t dr_lof_workspace_bytes(int64_t n);
+int dr_lof_flag(dr_ctx* ctx, const double* col, int64_t n, int k, int64_t row_begin, int64_t row_count,
+                uint32_t* bitmap, double* out_lof, int64_t* out_flagged, void* workspace, int64_t workspace_bytes,
+                void* stream);
+
 /* PoorModel (model.py:44-61): constant fill of the listed tile rows. */
 int dr_tile_fill_i32(dr_ctx* ctx, int32_t* tile, int n_cols, int col, const int32_t* cells, int64_t n_cells,
                      int32_t value, void* stream);

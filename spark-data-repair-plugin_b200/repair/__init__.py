@@ -3,7 +3,8 @@
 sm_100a CUDA (``libb200repair.so``) instead of Spark SQL + pandas UDFs."""
 from .api import Delphi  # noqa: F401
 from .errors import (ConstraintErrorDetector, DomainValues, ErrorDetector,  # noqa: F401
-                     GaussianOutlierErrorDetector, NullErrorDetector, RegExErrorDetector)
+                     GaussianOutlierErrorDetector, LOFOutlierErrorDetector, NullErrorDetector, RegExErrorDetector,
+                     ScikitLearnBackedErrorDetector, ScikitLearnBasedErrorDetector)
 from .model import RepairModel  # noqa: F401
 
 delphi = Delphi.getOrCreate()

@@ -75,6 +75,9 @@ _SIGNATURES = {
     "dr_lut_scan": (c_int, [c_void_p, c_void_p, c_int64, c_void_p, c_int32, c_void_p, c_void_p]),
     "dr_quartiles": (c_int, [c_void_p, c_void_p, c_int64, POINTER(c_double), POINTER(c_int64), c_void_p]),
     "dr_range_flag": (c_int, [c_void_p, c_void_p, c_int64, c_double, c_double, c_void_p, c_void_p]),
+    "dr_lof_workspace_bytes": (c_int64, [c_int64]),
+    "dr_lof_flag": (c_int, [c_void_p, c_void_p, c_int64, c_int, c_int64, c_int64, c_void_p, c_void_p,
+                            POINTER(c_int64), c_void_p, c_int64, c_void_p]),
     "dr_dc_const": (c_int, [c_void_p, _PP, POINTER(c_int32), POINTER(c_int32), c_int, c_int64, c_void_p, c_void_p]),
     "dr_dc_fd_build": (c_int, [c_void_p, _PP, POINTER(c_int64), c_int, c_void_p, c_int64, c_int64, c_void_p,
                                c_void_p, c_void_p]),
@@ -301,6 +304,22 @@ class Context:
 
     def range_flag(self, col, n_rows, lower, upper, bitmap):
         self._check(self.lib.dr_range_flag(self._h, _dp(col), n_rows, lower, upper, _dp(bitmap), self._stream()))
+
+    def lof_workspace_bytes(self, n):
+        nbytes = int(self.lib.dr_lof_workspace_bytes(n))
+        if nbytes < 0:
+            raise NativeError("libb200repair: dr_lof_workspace_bytes({}) failed".format(n))
+        return nbytes
+
+    def lof_flag(self, col, n, k, row_begin, row_count, bitmap, workspace, out_lof=None, count=False):
+        """Exact 1-D LOF of col[:n] (the whole column); rows in [row_begin, row_begin + row_count) with
+        lof > 1.5 set bit (row - row_begin) of `bitmap`.  workspace: device uint8 tensor of at least
+        lof_workspace_bytes(n) bytes.  With count=True, returns the number of flagged rows (synchronises)."""
+        flagged = c_int64()
+        self._check(self.lib.dr_lof_flag(self._h, _dp(col), n, k, row_begin, row_count, _dp(bitmap), _dp(out_lof),
+                                         byref(flagged) if count else None, _dp(workspace), workspace.numel(),
+                                         self._stream()))
+        return int(flagged.value) if count else None
 
     def dc_const(self, cols, ops, args, n_rows, row_bitmap):
         cp, _k = _ptr_array([c.data_ptr() for c in cols])
@@ -536,7 +555,7 @@ def _profiled(name, fn):
 
 
 for _name in ("widen_u8", "h2d_copy", "d2h_copy", "index_presence", "index_remap", "ids_unique", "gather_i64", "valid_bits",
-              "scan_hist", "lut_scan", "quartiles", "range_flag", "dc_const", "dc_fd_build", "dc_fd_flag", "bitmap_or",
+              "scan_hist", "lut_scan", "quartiles", "range_flag", "lof_flag", "dc_const", "dc_fd_build", "dc_fd_flag", "bitmap_or",
               "bitmap_andnot", "bitmap_count", "bitmap_count_many", "bitmap_to_rows_async", "bitmaps_to_rows_many", "bitmap_to_rows", "bitmap_rows_after_count", "tile_null_bitmaps", "changed_bitmap", "bitmap_gather", "bitmap_clear_rows", "discretize",
               "pair_presence", "cooc", "cooc_skip", "key_presence", "key_flag", "dc_exists", "combine_counts", "dc_lt_flag",
               "dc_hash_build", "dc_hash_flag", "domain_score", "domain_prune", "gather_rows_masked", "tile_null_bitmap", "gather",

@@ -593,6 +593,65 @@ class Engine:
                 bitmaps[a] = self.new_bitmap()
             self.ctx.range_flag(self.dt.val(a), self.n_rows, lower, upper, bitmaps[a])
 
+    def _global_values(self, a):
+        """-> (device float64 values of continuous attribute `a` over the whole table, first global row of this
+        shard).  Sharded: one all-gather, rank order."""
+        v = self.dt.val(a)[:self.n_rows]
+        if self.dist is None:
+            return v, 0
+        col, counts = self.dist.all_gather_rows(v.contiguous())
+        return col, int(sum(counts[:self.dist.rank]))
+
+    def detect_lof(self, targets, bitmaps, k=20):
+        """LOFOutlierErrorDetector (errors.py:302-312): exact one-dimensional local outlier factor of every
+        continuous target, k = min(20, n - 1) like LocalOutlierFactor's default.  Sharded, every rank scores the
+        gathered global column and sets the bits of its own rows only, so the union equals the one-GPU result."""
+        ws = None
+        for a in self.table.continuous_attrs:
+            if a not in targets:
+                continue
+            col, row_begin = self._global_values(a)
+            n = int(col.shape[0])
+            if n < 2:
+                continue
+            if ws is None:
+                ws = self.torch.empty(self.ctx.lof_workspace_bytes(n), dtype=self.torch.uint8, device=self.device)
+            if a not in bitmaps:
+                bitmaps[a] = self.new_bitmap()
+            self.ctx.lof_flag(col, n, min(k, n - 1), row_begin, self.n_rows, bitmaps[a], ws)
+
+    def detect_sklearn(self, targets, bitmaps, factory):
+        """ScikitLearnBackedErrorDetector (errors.py:219-245): the user's estimator, built by `factory`, runs on
+        the host over the global column with NULLs filled by the median (errors.py:237-238); `fit_predict` < 0
+        flags a row.  Sharded, only rank 0 fits and one broadcast hands every rank the same answer."""
+        import pandas as pd
+        torch = self.torch
+        for a in self.table.continuous_attrs:
+            if a not in targets:
+                continue
+            col, row_begin = self._global_values(a)
+            n = int(col.shape[0])
+            flags = torch.zeros(n, dtype=torch.uint8, device=self.device)
+            if self.dist is None or self.dist.rank == 0:
+                vals = col.cpu().numpy()
+                valid = ~np.isnan(vals)
+                if n >= 2 and valid.any():
+                    pdf = pd.DataFrame({a: vals})
+                    pred = np.asarray(factory().fit_predict(pdf[[a]].fillna(np.median(vals[valid]))))
+                    flags.copy_(torch.from_numpy((pred < 0).astype(np.uint8)))
+            if self.dist is not None:
+                td, group = self.dist.td, self.dist.group
+                td.broadcast(flags, src=td.get_global_rank(group, 0) if group is not None else 0, group=group)
+            mine = flags[row_begin:row_begin + self.n_rows].cpu().numpy()
+            if not mine.any():
+                continue
+            words = np.zeros(self.n_words * 4, dtype=np.uint8)
+            packed = np.packbits(mine, bitorder="little")
+            words[:len(packed)] = packed
+            if a not in bitmaps:
+                bitmaps[a] = self.new_bitmap()
+            self.ctx.bitmap_or(bitmaps[a], torch.from_numpy(words.view(np.int32)).to(self.device), self.n_rows)
+
     def bitmaps_from_cells(self, positions, attrs):
         """User-supplied error cells (setErrorCells) -> bitmaps, built on the host."""
         out = {}
@@ -848,7 +907,7 @@ class Engine:
 
     # ---- ErrorModel.detect -----------------------------------------------------------------------
     def detect(self, detectors, targets, discrete_thres, opts, given_cells=None):
-        """detectors: list of dicts {"type": null|domain|regex|constraint|outlier, ...}
+        """detectors: list of dicts {"type": null|domain|regex|constraint|outlier|lof|sklearn, ...}
         given_cells: optional (positions, attrs) supplied by setErrorCells.
 
         Pass structure (the same on one GPU and on G shards; exchange() is the only cross-GPU step):
@@ -900,6 +959,10 @@ class Engine:
                     self.detect_constraints(det.get("path", ""), det.get("constraints", ""), tg, bitmaps, ex1, after)
                 elif kind == "outlier":
                     self.detect_outliers(tg, bitmaps, det.get("approx", False))
+                elif kind == "lof":
+                    self.detect_lof(tg, bitmaps)
+                elif kind == "sklearn":
+                    self.detect_sklearn(tg, bitmaps, det["factory"])
                 else:
                     raise ValueError("unknown detector type: {}".format(kind))
         # local 1 (cont.): one fused pass for the NULL bits of the discretised targets + every histogram,

@@ -1,12 +1,12 @@
 """Error detectors: same class names, constructors and ``setUp(...).detect()`` protocol as the
-reference (``python/repair/errors.py:37-190``), evaluated by CUDA scans instead of Spark SQL.
+reference (``python/repair/errors.py:37-312``), evaluated by CUDA scans instead of Spark SQL.
 
 A detector is a small value object; ``spec()`` lowers it to the dict the device pipeline
 (``engine.Engine.detect``) consumes.  ``detect()`` on a detector that was ``setUp`` against an
 input registered in the catalog returns a pandas frame ``(row_id, attribute)``.
 """
 from abc import ABCMeta, abstractmethod
-from typing import Any, Dict, List, Optional
+from typing import Any, Callable, Dict, List, Optional
 
 from .utils import get_option_value
 
@@ -116,6 +116,66 @@ class GaussianOutlierErrorDetector(ErrorDetector):
 
     def spec(self):
         return {"type": "outlier", "approx": self.approx_enabled}
+
+
+class ScikitLearnBasedErrorDetector(ErrorDetector):
+    """Per-column outlier detection over the continuous targets (errors.py:193-279).  The reference scores
+    random partitions of tables with at least `parallel_mode_threshold` rows; here the whole column is scored
+    at any size, so `parallel_mode_threshold` and `num_parallelism` are validated and kept but change
+    nothing."""
+
+    def __init__(self, parallel_mode_threshold: int = 10000, num_parallelism: Optional[int] = None) -> None:
+        ErrorDetector.__init__(self)
+
+        if num_parallelism is not None and int(num_parallelism) <= 0:
+            raise ValueError(f'`num_parallelism` must be positive, got {num_parallelism}')
+
+        self.parallel_mode_threshold = parallel_mode_threshold
+        self.num_parallelism = num_parallelism
+
+    def __str__(self) -> str:
+        return f'{self.__class__.__name__}()'
+
+    # An instance with a scikit-learn-like `fit_predict(X)` returning 1 (inlier) or -1 (outlier) per row.
+    @abstractmethod
+    def _outlier_detector_impl(self) -> Any:
+        pass
+
+
+class ScikitLearnBackedErrorDetector(ScikitLearnBasedErrorDetector):
+    """A user-supplied estimator, fitted on the host per target column (NULLs filled with the median)."""
+
+    def __init__(self, error_detector_cls: Callable[[], Any], parallel_mode_threshold: int = 10000,
+                 num_parallelism: Optional[int] = None) -> None:
+        ScikitLearnBasedErrorDetector.__init__(self, parallel_mode_threshold, num_parallelism)
+
+        if not hasattr(error_detector_cls, "__call__"):
+            raise ValueError('`error_detector_cls` should be callable')
+        if not hasattr(error_detector_cls(), "fit_predict"):
+            raise ValueError('An instance that `error_detector_cls` returns should have a `fit_predict` method')
+
+        self.error_detector_cls = error_detector_cls
+
+    def _outlier_detector_impl(self) -> Any:
+        return self.error_detector_cls()
+
+    def spec(self):
+        return {"type": "sklearn", "factory": self._outlier_detector_impl}
+
+
+class LOFOutlierErrorDetector(ScikitLearnBasedErrorDetector):
+    """LocalOutlierFactor(novelty=False) per continuous target, computed exactly on the GPU (dr_lof_flag):
+    k = min(20, n - 1), a cell is an error iff its local outlier factor exceeds 1.5."""
+
+    def __init__(self, parallel_mode_threshold: int = 10000, num_parallelism: Optional[int] = None) -> None:
+        ScikitLearnBasedErrorDetector.__init__(self, parallel_mode_threshold, num_parallelism)
+
+    def _outlier_detector_impl(self) -> Any:
+        from sklearn.neighbors import LocalOutlierFactor
+        return LocalOutlierFactor(novelty=False)
+
+    def spec(self):
+        return {"type": "lof"}
 
 
 class ErrorModelOptions:

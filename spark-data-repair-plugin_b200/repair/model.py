@@ -1058,6 +1058,10 @@ def detect_with(detector):
             engine.detect_constraints(spec["path"], spec["constraints"], targets, bitmaps)
         elif kind == "outlier":
             engine.detect_outliers(targets, bitmaps, spec.get("approx", False))
+        elif kind == "lof":
+            engine.detect_lof(targets, bitmaps)
+        elif kind == "sklearn":
+            engine.detect_sklearn(targets, bitmaps, spec["factory"])
         ids, attrs = [], []
         for a in table.names:
             if a in bitmaps:
